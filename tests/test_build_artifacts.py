@@ -2,7 +2,6 @@
 memory instructions. Reads the ptxas logs / objects `make -C jolt_b200/csrc` leaves in-tree; skipped before a build."""
 import pathlib
 import re
-import shutil
 import subprocess
 
 import pytest
@@ -64,8 +63,12 @@ def test_resident_kernels_fit_two_blocks_per_sm():
 
 
 def test_streaming_kernels_use_256_bit_memory_instructions():
+    from __graft_entry__ import find_cuda_tool
     obj = CSRC / "member.o"
-    cuobjdump = shutil.which("cuobjdump")
+    try:
+        cuobjdump = find_cuda_tool("cuobjdump")
+    except FileNotFoundError:
+        cuobjdump = None
     if not obj.exists() or cuobjdump is None:
         pytest.skip("member.o or cuobjdump not available")
     fn = "_ZN2jb18fused_round_kernelILi2ELi1ELi1ELb1ELb1ELb1ELi256ELi2ELb0EEEvNS_9TablePtrsEmNS_10BindScalarENS_8RoundOutE"
