@@ -110,32 +110,22 @@ int jbi::eq_build(jb_ctx* c, const uint64_t* r, size_t nvars, const uint64_t* sc
     int st = c->dev_alloc((void**)&d_prefix, ((size_t)1 << hi_vars) * 32);
     if (st == JB_OK) st = c->dev_alloc((void**)&d_low8, 256 * 32);
     if (st == JB_OK) st = eq_build(c, r, hi_vars, scale, d_prefix);
-    // layout (JB_EQ_LAYOUT: 0 (default) = the 3 register variables FIRST in the block, a warp's store covers 1 KiB;
-    // 1 = LAST: 8 consecutive outputs per thread. ncu A/B at 2^26 (profiles/r02_eq_store_ab.md): both write 2.0 x the
-    // table to DRAM whatever the store flavour, layout 0 is ~7 % faster)
-    const bool low3 = c->eq_layout != 0;
-    if (st == JB_OK) st = eq_build(c, r + 4 * (hi_vars + (low3 ? 0 : 3)), 8, nullptr, d_low8);
+    // the block's first 3 variables are expanded in registers (eq_stream_kernel), its last 8 come from low8
+    if (st == JB_OK) st = eq_build(c, r + 4 * (hi_vars + 3), 8, nullptr, d_low8);
     if (st == JB_OK) {
         int tix = c->timing_begin(3, (uint64_t)1 << nvars, 1);
-        const uint64_t* r3 = r + 4 * (hi_vars + (low3 ? 8 : 0));
+        const uint64_t* r3 = r + 4 * hi_vars;
         bool hi4 = true;  // all three register-stage variables are 125-bit challenges [0,0,lo,hi]
         for (int j = 0; j < 3; ++j) hi4 = hi4 && r3[4 * j] == 0 && r3[4 * j + 1] == 0;
         const unsigned g = (unsigned)((size_t)1 << hi_vars);
-        // tables beyond what L2 can usefully keep are streamed out with evict-first stores (JB_EQ_STORE=0/1 forces)
-        const bool cs = c->eq_store_mode < 0 ? nvars >= 22 : c->eq_store_mode == 1;
+        // tables beyond what L2 can usefully keep are streamed out with evict-first stores
+        const bool cs = nvars >= 22;
         const EqVars v3 = eq_vars(r3, 3, nullptr);
-#define JB_EQ_LAUNCH(H, C, L) eq_stream_kernel<H, C, L><<<g, 256, 0, c->stream>>>(d_prefix, v3, d_low8, d_out)
-        if (low3) {
-            if (hi4 && cs) JB_EQ_LAUNCH(true, true, true);
-            else if (hi4) JB_EQ_LAUNCH(true, false, true);
-            else if (cs) JB_EQ_LAUNCH(false, true, true);
-            else JB_EQ_LAUNCH(false, false, true);
-        } else {
-            if (hi4 && cs) JB_EQ_LAUNCH(true, true, false);
-            else if (hi4) JB_EQ_LAUNCH(true, false, false);
-            else if (cs) JB_EQ_LAUNCH(false, true, false);
-            else JB_EQ_LAUNCH(false, false, false);
-        }
+#define JB_EQ_LAUNCH(H, C) eq_stream_kernel<H, C><<<g, 256, 0, c->stream>>>(d_prefix, v3, d_low8, d_out)
+        if (hi4 && cs) JB_EQ_LAUNCH(true, true);
+        else if (hi4) JB_EQ_LAUNCH(true, false);
+        else if (cs) JB_EQ_LAUNCH(false, true);
+        else JB_EQ_LAUNCH(false, false);
 #undef JB_EQ_LAUNCH
         c->timing_end(tix);
         c->launches++;
@@ -194,15 +184,8 @@ static int ctx_create_impl(int device, bool borrow, void* cuda_stream, jb_ctx** 
     cudaDeviceProp prop;
     cudaGetDeviceProperties(&prop, device);
     c->sm_count = prop.multiProcessorCount;
-    if (const char* sh = std::getenv("JB_FUSED_SHAPE")) c->fused_shape = std::atoi(sh);  // tuning knob
     if (std::getenv("JB_NO_TAIL")) c->use_tail = false;  // diagnostics: one launch per round all the way down
-    if (const char* ml = std::getenv("JB_RESIDENT_MAX_LOG")) c->resident_max_log = std::atoi(ml);
-    if (const char* sp = std::getenv("JB_STATIC_PCT")) c->resident_static_pct = std::max(0, std::min(100, std::atoi(sp)));
     if (const char* ts = std::getenv("JB_RESIDENT_TIMEOUT_S")) c->resident_timeout_cycles = (long long)(std::atof(ts) * 1.9e9);
-    if (std::getenv("JB_EVAL_TMA")) c->eval_tma = true;
-    if (std::getenv("JB_NO_LOOKAHEAD")) c->lookahead = false;
-    if (const char* es = std::getenv("JB_EQ_STORE")) c->eq_store_mode = std::atoi(es);
-    if (const char* el = std::getenv("JB_EQ_LAYOUT")) c->eq_layout = std::atoi(el);  // diagnostics: every round waits for its own answer
     // A kernel-replaying profiler (ncu) or a serialising tool (compute-sanitizer, nsys CUDA trace) cannot
     // run a kernel that waits for host commands; under CUDA injection keep one launch per round.
     {

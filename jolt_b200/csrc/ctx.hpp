@@ -80,13 +80,7 @@ struct jb_ctx {
     std::vector<TailRes> tail_pool;
     uint64_t diag_wait_ns = 0, diag_waits = 0;  // host time spent waiting for round results
     bool use_tail = true;           // resident kernel service (off under profilers / JB_NO_TAIL: one launch per round)
-    bool eval_tma = false;          // A/B: TMA-staged variant of the degree-2 eval-only sweep (JB_EVAL_TMA=1)
-    int eq_layout = 0;              // eq stream kernel: 0 = a warp writes 1 KiB runs (a thread's outputs 8 KiB apart), 1 = a thread's 8 outputs consecutive
-    int eq_store_mode = -1;         // eq table stores: -1 auto, 0 default caching, 1 streaming (evict-first)
-    int resident_static_pct = 75;  // big resident passes: statically laid-out share of the range (JB_STATIC_PCT; 100 = all)
     long long resident_timeout_cycles = 20000000000LL;  // a resident kernel gives its SMs back after this long without a command
-    bool lookahead = true;          // answer thin rounds from the previous answer's lookahead sums (JB_NO_LOOKAHEAD: off)
-    int resident_max_log = 40;      // a member may enter resident service when log2(len) <= this (JB_RESIDENT_MAX_LOG)
     std::vector<ResidentRun*> runs; // live resident kernels of this context
     // diagnostics: per round of the last completed run: device %globaltimer at command decode / after the fold,
     // host CLOCK_MONOTONIC at post / at receipt (ns)
@@ -97,7 +91,6 @@ struct jb_ctx {
     // (<= half the device) runs. The members they served continue with one launch per round.
     void quiesce_resident(bool all = false);
     bool has_exclusive_run() const;
-    int fused_shape = 0;            // fused-kernel occupancy shape (see launch_fused)
     bool verify_rounds = false;     // compute s(1) and check s(0)+s(1)==claim instead of deriving s(1)
     uint64_t* d_small = nullptr;    // device staging
     uint64_t* h_small = nullptr;    // pinned host staging

@@ -15,7 +15,6 @@
 #include "member.hpp"
 #include "resident.cuh"
 #include "sumcheck_host.hpp"
-#include "tma_ab.cuh"
 
 using namespace jb;
 using namespace jbi;
@@ -27,18 +26,19 @@ constexpr int JB_SLOT_U64 = 128;
 
 namespace {
 
-template <int M, int P, int ORDER, bool BIND, bool HI4, bool SKIP1, int BLOCK, int MINB>
-int launch_fused_mb(jb_ctx* c, const TablePtrs& tp, size_t pairs, const BindScalar& s, RoundOut out) {
-    auto kernel = fused_round_kernel<M, P, ORDER, BIND, HI4, SKIP1, BLOCK, MINB>;
-    constexpr size_t smem = FusedShape<M, SKIP1>::smem_bytes(BLOCK);
+// One launch per round, 256 threads x 2 blocks per SM. WEIGHTED: the split-eq pass (s(1) from the claim).
+template <int M, int P, int ORDER, bool BIND, bool HI4, bool SKIP1, bool WEIGHTED = false>
+int launch_fused(jb_ctx* c, const TablePtrs& tp, size_t pairs, const BindScalar& s, RoundOut out) {
+    auto kernel = fused_round_kernel<M, P, ORDER, BIND, HI4, SKIP1, 256, 2, WEIGHTED>;
+    constexpr size_t smem = FusedShape<M, SKIP1>::smem_bytes(256);
     static int per_sm = [&] {
         cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         int nb = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kernel, BLOCK, smem) != cudaSuccess || nb < 1) nb = 1;
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kernel, 256, smem) != cudaSuccess || nb < 1) nb = 1;
         return nb;
     }();
     // grid-stride over whole waves of resident blocks; tiny rounds take one (small) block
-    size_t need = (pairs + BLOCK - 1) / BLOCK;
+    size_t need = (pairs + 255) / 256;
     size_t resident = (size_t)c->sm_count * per_sm;
     size_t grid = need < resident ? need : resident;
     if (grid < 1) grid = 1;
@@ -48,83 +48,19 @@ int launch_fused_mb(jb_ctx* c, const TablePtrs& tp, size_t pairs, const BindScal
     out.partial = c->d_partial;
     int tix = c->timing_begin(BIND ? 0 : 2, pairs, M * P);
     // latency path: a round of <= 32 pairs runs as one warp (no barriers, no shared-memory stage)
-    const unsigned block = pairs <= 32 ? 32u : (unsigned)BLOCK;
-    kernel<<<(unsigned)grid, block, smem, c->stream>>>(tp, pairs, s, out);
-    c->timing_end(tix);
-    c->launches++;
-    return c->check(cudaGetLastError(), "fused_round_kernel launch");
-}
-
-// A/B (JB_EVAL_TMA=1): the degree-2 eval-only sweep with its evaluation blocks staged by the TMA unit (tma_ab.cuh)
-template <int ORDER>
-int launch_eval2_tma(jb_ctx* c, const TablePtrs& tp, size_t pairs, RoundOut out) {
-    auto kernel = eval2_tma_kernel<ORDER>;
-    constexpr size_t smem = TmaShape::smem_bytes;
-    static int per_sm = [&] {
-        cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        int nb = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kernel, TMA_THREADS, smem) != cudaSuccess || nb < 1) nb = 1;
-        return nb;
-    }();
-    size_t need = (pairs + TMA_TILE - 1) / TMA_TILE;
-    size_t resident = (size_t)c->sm_count * per_sm;
-    size_t grid = need < resident ? need : resident;
-    if (grid < 1) grid = 1;
-    int st = c->ensure_partial(grid * 2);
-    if (st != JB_OK) return st;
-    out.partial = c->d_partial;
-    int tix = c->timing_begin(2, pairs, 2);
-    kernel<<<(unsigned)grid, TMA_THREADS, smem, c->stream>>>(tp, pairs, out);
-    c->timing_end(tix);
-    c->launches++;
-    return c->check(cudaGetLastError(), "eval2_tma_kernel launch");
-}
-
-template <int M, int P, int ORDER, bool BIND, bool HI4, bool SKIP1>
-int launch_fused(jb_ctx* c, const TablePtrs& tp, size_t pairs, const BindScalar& s, const RoundOut& out) {
-    if constexpr (M == 2 && P == 1 && !BIND && SKIP1) {
-        if (c->eval_tma && pairs >= 4096) return launch_eval2_tma<ORDER>(c, tp, pairs, out);
-    }
-    // occupancy shapes (tuning knob JB_FUSED_SHAPE): 0 = 256 threads x 2 blocks (128 registers),
-    // 1 = 128 threads x 5 blocks (<= 102 registers, 20 warps/SM)
-    if constexpr (M == 2 && P == 1) {
-        if (c->fused_shape == 1) return launch_fused_mb<M, P, ORDER, BIND, HI4, SKIP1, 128, 5>(c, tp, pairs, s, out);
-    }
-    return launch_fused_mb<M, P, ORDER, BIND, HI4, SKIP1, 256, 2>(c, tp, pairs, s, out);
-}
-
-// weighted (split-eq) passes: s(1) from the claim, 256 x 2
-template <int M, int ORDER, bool BIND, bool HI4>
-int launch_weighted(jb_ctx* c, const TablePtrs& tp, size_t pairs, const BindScalar& s, RoundOut out) {
-    auto kernel = fused_round_kernel<M, 1, ORDER, BIND, HI4, true, 256, 2, true>;
-    constexpr size_t smem = FusedShape<M, true>::smem_bytes(256);
-    static int per_sm = [&] {
-        cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        int nb = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kernel, 256, smem) != cudaSuccess || nb < 1) nb = 1;
-        return nb;
-    }();
-    size_t need = (pairs + 255) / 256;
-    size_t resident = (size_t)c->sm_count * per_sm;
-    size_t grid = need < resident ? need : resident;
-    if (grid < 1) grid = 1;
-    int st = c->ensure_partial(grid * M);
-    if (st != JB_OK) return st;
-    out.partial = c->d_partial;
-    int tix = c->timing_begin(BIND ? 0 : 2, pairs, M);
     const unsigned block = pairs <= 32 ? 32u : 256u;
     kernel<<<(unsigned)grid, block, smem, c->stream>>>(tp, pairs, s, out);
     c->timing_end(tix);
     c->launches++;
-    return c->check(cudaGetLastError(), "fused_round_kernel (weighted) launch");
+    return c->check(cudaGetLastError(), WEIGHTED ? "fused_round_kernel (weighted) launch" : "fused_round_kernel launch");
 }
 
 template <int M, int ORDER>
 int dispatch_weighted1(jb_ctx* c, const TablePtrs& tp, size_t pairs, bool bind, bool hi4, const BindScalar& s,
                        const RoundOut& out) {
-    if (!bind) return launch_weighted<M, ORDER, false, false>(c, tp, pairs, s, out);
-    return hi4 ? launch_weighted<M, ORDER, true, true>(c, tp, pairs, s, out)
-               : launch_weighted<M, ORDER, true, false>(c, tp, pairs, s, out);
+    if (!bind) return launch_fused<M, 1, ORDER, false, false, true, true>(c, tp, pairs, s, out);
+    return hi4 ? launch_fused<M, 1, ORDER, true, true, true, true>(c, tp, pairs, s, out)
+               : launch_fused<M, 1, ORDER, true, false, true, true>(c, tp, pairs, s, out);
 }
 
 int dispatch_weighted(jb_ctx* c, int m, int order, const TablePtrs& tp, size_t pairs, bool bind, bool hi4, const BindScalar& s,
@@ -441,7 +377,7 @@ static void answer_values(const jb_member* mem, const ResConsumed& info, const u
 
 // A thin answer also determines the NEXT round's polynomial as a function of the challenge that round binds.
 static void harvest_lookahead(jb_member* mem, const ResConsumed& info, const uint64_t* lanes) {
-    if ((info.act == RES_ACT_EVAL || info.act == RES_ACT_BIND_EVAL) && info.thin && info.nprime >= 4 && mem->ctx->lookahead) {
+    if ((info.act == RES_ACT_EVAL || info.act == RES_ACT_BIND_EVAL) && info.thin && info.nprime >= 4) {
         jb_wide_lanes_reduce_host(lanes, 6, mem->look);
         mem->look_ok = true;
         mem->look_round = info.round + 1;
@@ -493,7 +429,7 @@ static int run_round(jb_ctx* c, ResidentRun* run, RunItem* items, int n, const u
     bool hit[RES_MAX_MEMBERS], need_now = false;
     for (int i = 0; i < n && !lost; ++i) {
         jb_member* m = items[i].mem;
-        hit[i] = c->lookahead && items[i].bind && m->look_ok && m->look_round == items[i].round && m->m == 2;
+        hit[i] = items[i].bind && m->look_ok && m->look_round == items[i].round && m->m == 2;
         if (hit[i]) lookahead_values(m, items[i].bind, vals[i]);
         else need_now = true;
     }
@@ -871,8 +807,7 @@ static int sharded_prove_round(jb_member* mem, const uint64_t* bind, size_t roun
             // the peers' shards and sweeps the gathered tables - no kernel exit, no NCCL call; from here on this
             // member proves its remaining rounds un-sharded (identically on every rank)
             const bool skip1g = claim != nullptr && !c->verify_rounds;
-            if (bind && skip1g && mem->run && len_after == mem->gather_len && resident_gather_fits(c, mem, len_after) &&
-                !std::getenv("JB_NCCL_GATHER")) {
+            if (bind && skip1g && mem->run && len_after == mem->gather_len && resident_gather_fits(c, mem, len_after)) {
                 int st = resident_member_prove(mem, bind, claim, round, false, out_evals, true);
                 if (st == JB_OK) {
                     mem->rounds_done--;  // (the caller counts sharded rounds)

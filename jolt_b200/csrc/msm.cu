@@ -19,13 +19,11 @@
 // (mod.rs:205) becomes a one-time normalisation at upload.
 #include <cuda_runtime.h>
 
-#include <cstdlib>
 #include <cstring>
 #include <vector>
 
 #include "ctx.hpp"
 #include "ec.cuh"
-#include "msm_affine.cuh"
 #include "small_scalar.cuh"
 
 using namespace jb;
@@ -35,14 +33,8 @@ namespace {
 // buckets per reduction segment: one thread walks a segment (2 general additions per bucket) and then multiplies the
 // segment's plain sum by its first bucket number (double-and-add, ~330 products): the multiplication is per SEGMENT, so
 // short segments cost work (measured at 2^20 / 2^24 terms, precomputed SRS: 8 buckets 0.88 / 3.76 ms, 16 buckets
-// 0.55 / 2.38 ms). JB_MSM_SEG overrides (A/B).
+// 0.55 / 2.38 ms).
 int msm_seg_size(int buckets) {
-    static const int env = [] {
-        const char* e = getenv("JB_MSM_SEG");
-        const int x = e ? atoi(e) : 0;
-        return x >= 2 && x <= 256 ? x : 0;
-    }();
-    if (env) return env;
     return buckets >= (1 << 21) ? 64 : 16;  // 2^24 terms (2^21 buckets): 16 / 32 / 64 = 40.6 / 40.0 / 39.7 ms per MSM; 2^20 terms: 3.17 / 3.26 / 3.61
 }
 
@@ -249,24 +241,17 @@ __device__ __forceinline__ void block_exclusive_scan2(unsigned int& a, unsigned 
     __syncthreads();
 }
 
-// pad_shift = L > 0 (batched-affine levels, msm_affine.cuh): the point offsets are scanned over counts padded to a
-// multiple of 2^L and the tasks are planned over the ceil(cnt / 2^L) points a bucket has left after L halvings.
 __global__ void __launch_bounds__(1024) msm_scan_local_kernel(unsigned int* hist, unsigned int* offsets, unsigned int* toff,
-                                                              size_t total, unsigned int* block_sums, unsigned maxq,
-                                                              unsigned pad_shift) {
+                                                              size_t total, unsigned int* block_sums, unsigned maxq) {
     __shared__ unsigned int sm_a[32], sm_b[32];
     const size_t base = (size_t)blockIdx.x * SCAN_PER_BLOCK + (size_t)threadIdx.x * 4;
     unsigned int c[4] = {0, 0, 0, 0};
 #pragma unroll
     for (int k = 0; k < 4; ++k)
         if (base + k < total) c[k] = hist[base + k];
-    const unsigned pad_mask = (1u << pad_shift) - 1u;
     unsigned int q[4];
 #pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        c[k] = (c[k] + pad_mask) & ~pad_mask;
-        q[k] = chunk_count(c[k] >> pad_shift, maxq);
-    }
+    for (int k = 0; k < 4; ++k) q[k] = chunk_count(c[k], maxq);
     unsigned int sa = c[0] + c[1] + c[2] + c[3], sb = q[0] + q[1] + q[2] + q[3], ta, tb;
     block_exclusive_scan2(sa, sb, sm_a, sm_b, ta, tb);
 #pragma unroll
@@ -329,7 +314,7 @@ __device__ __forceinline__ int task_len_bin(unsigned cnt, unsigned maxq) {
 // memory, so the 256 global counters see one atomic per (block, non-empty bin) instead of one per warp and bin.
 constexpr int MSM_TASK_BLOCKS = 592;
 __global__ void __launch_bounds__(256) msm_len_hist_kernel(const unsigned int* offsets, const unsigned int* toff, size_t nbuckets,
-                                                           unsigned maxq, unsigned int* len_hist, unsigned shift) {
+                                                           unsigned maxq, unsigned int* len_hist) {
     __shared__ unsigned int cnt_s[MSM_LEN_BINS];
     cnt_s[threadIdx.x] = 0;
     __syncthreads();
@@ -337,7 +322,7 @@ __global__ void __launch_bounds__(256) msm_len_hist_kernel(const unsigned int* o
     const size_t b0 = (size_t)blockIdx.x * per, b1 = b0 + per < nbuckets ? b0 + per : nbuckets;
     for (size_t b = b0 + threadIdx.x; b < b1; b += blockDim.x) {
         const unsigned q = toff[b + 1] - toff[b];
-        if (q) atomicAdd(&cnt_s[task_len_bin((offsets[b + 1] - offsets[b]) >> shift, maxq)], q);
+        if (q) atomicAdd(&cnt_s[task_len_bin(offsets[b + 1] - offsets[b], maxq)], q);
     }
     __syncthreads();
     if (cnt_s[threadIdx.x]) atomicAdd(&len_hist[threadIdx.x], cnt_s[threadIdx.x]);
@@ -345,7 +330,7 @@ __global__ void __launch_bounds__(256) msm_len_hist_kernel(const unsigned int* o
 // len_hist: [0, 256) task counts per bin (read), [256, 512) cursors (zero on entry)
 __global__ void __launch_bounds__(256) msm_tasks_kernel(const unsigned int* offsets, const unsigned int* toff, size_t nbuckets,
                                                         unsigned maxq, unsigned int* len_hist, uint32_t* task_bucket,
-                                                        uint32_t* order, unsigned shift) {
+                                                        uint32_t* order) {
     __shared__ unsigned int bin_base[MSM_LEN_BINS], cnt_s[MSM_LEN_BINS], tmp[MSM_LEN_BINS];
     const int k = threadIdx.x;
     {   // exclusive scan of the 256 bin counts (Hillis-Steele in shared memory)
@@ -366,7 +351,7 @@ __global__ void __launch_bounds__(256) msm_tasks_kernel(const unsigned int* offs
     const size_t b0 = (size_t)blockIdx.x * per, b1 = b0 + per < nbuckets ? b0 + per : nbuckets;
     for (size_t b = b0 + k; b < b1; b += blockDim.x) {  // this block's tasks per bin
         const unsigned q = toff[b + 1] - toff[b];
-        if (q) atomicAdd(&cnt_s[task_len_bin((offsets[b + 1] - offsets[b]) >> shift, maxq)], q);
+        if (q) atomicAdd(&cnt_s[task_len_bin(offsets[b + 1] - offsets[b], maxq)], q);
     }
     __syncthreads();
     if (cnt_s[k]) bin_base[k] += atomicAdd(&len_hist[MSM_LEN_BINS + k], cnt_s[k]);  // this block's share of bin k
@@ -375,7 +360,7 @@ __global__ void __launch_bounds__(256) msm_tasks_kernel(const unsigned int* offs
     for (size_t b = b0 + k; b < b1; b += blockDim.x) {
         const unsigned t0 = toff[b], q = toff[b + 1] - t0;
         if (!q) continue;
-        const int bin = task_len_bin((offsets[b + 1] - offsets[b]) >> shift, maxq);
+        const int bin = task_len_bin(offsets[b + 1] - offsets[b], maxq);
         const unsigned pos = bin_base[bin] + atomicAdd(&cnt_s[bin], q);
         for (unsigned j = 0; j < q; ++j) {
             task_bucket[t0 + j] = (uint32_t)b;
@@ -455,19 +440,16 @@ __global__ void __launch_bounds__(256) msm_scatter_kernel(const uint32_t* digits
 // ---- 4. bucket accumulation: the hot kernel. One thread per task (a chunk of one bucket's list). A
 //         single-chunk bucket is written straight to `buckets`; chunks of a split bucket go to `partial`
 //         and are folded by msm_combine_kernel. --------------------------------------------------------
-// DIRECT (after the batched-affine levels): `bases` is the level-L point array, bucket b owns its entries
-// [offsets[b] >> shift, offsets[b + 1] >> shift) - affine points or the identity (0, 0) - and there is no index list.
-template <bool DIRECT>
 __global__ void __launch_bounds__(128) msm_accumulate_kernel(const uint64_t* bases, const uint32_t* sorted,
                                                              const unsigned int* offsets, const unsigned int* toff,
                                                              const uint32_t* task_bucket, const uint32_t* order,
                                                              size_t nbuckets, uint64_t* buckets, uint64_t* partial,
-                                                             unsigned maxq, unsigned shift) {
+                                                             unsigned maxq) {
     const size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= toff[nbuckets]) return;
     const size_t t = order[k];  // tasks in length order (msm_tasks_kernel)
     const uint32_t b = task_bucket[t];
-    const unsigned int base = offsets[b] >> shift, cnt = (offsets[b + 1] >> shift) - base;
+    const unsigned int base = offsets[b], cnt = offsets[b + 1] - base;
     const unsigned int len = chunk_len(cnt, maxq), j = (unsigned int)t - toff[b];
     unsigned int lo = base + j * len;
     unsigned int hi = lo + len < base + cnt ? lo + len : base + cnt;
@@ -477,22 +459,16 @@ __global__ void __launch_bounds__(128) msm_accumulate_kernel(const uint64_t* bas
     uint32_t e_next = 0;
     Fq nx = Fq::zero(), ny = Fq::zero();
     auto fetch = [&](unsigned int at) {
-        if (DIRECT) {
-            nx = ld_elem_rw<Fq>(bases, 2 * (size_t)at);
-            ny = ld_elem_rw<Fq>(bases, 2 * (size_t)at + 1);
-        } else {
-            e_next = sorted[at];
-            nx = ld_elem<Fq>(bases, 2 * (size_t)(e_next & 0x7fffffffu));
-            ny = ld_elem<Fq>(bases, 2 * (size_t)(e_next & 0x7fffffffu) + 1);
-        }
+        e_next = sorted[at];
+        nx = ld_elem<Fq>(bases, 2 * (size_t)(e_next & 0x7fffffffu));
+        ny = ld_elem<Fq>(bases, 2 * (size_t)(e_next & 0x7fffffffu) + 1);
     };
     if (lo < hi) fetch(lo);
     for (unsigned int i = lo; i < hi; ++i) {
         const uint32_t e = e_next;
         const Fq px = nx, py = ny;
         if (i + 1 < hi) fetch(i + 1);
-        if (DIRECT && px.is_zero() && py.is_zero()) continue;  // a hole, or a pair that cancelled
-        xyzz_add_affine(acc, px, py, !DIRECT && (e >> 31) != 0);
+        xyzz_add_affine(acc, px, py, (e >> 31) != 0);
     }
     if (toff[b + 1] - toff[b] == 1) st_xyzz(buckets, b, acc);
     else st_xyzz(partial, t, acc);
@@ -854,11 +830,7 @@ int msm_device(jb_ctx* c, const Srs& srs, size_t offset, const void* d_scalars, 
     // wide window's bucket reduction (2^(c-1) buckets) to be in the noise
     // Small MSMs (the tail of HyperKZG's intermediate commitments, verifier-sized MSMs) use a second, tiny
     // table with 8-bit windows over the first bases: 128 buckets, no doubling chain - latency, not work.
-    static const size_t small_max = [] {  // JB_MSM_SMALL_MAX: largest MSM served by the 8-bit-window table (A/B)
-        const char* e = getenv("JB_MSM_SMALL_MAX");
-        const long v = e ? atol(e) : 4096;
-        return (size_t)(v > 0 ? v : 4096);
-    }();
+    constexpr size_t small_max = 4096;  // largest MSM served by the 8-bit-window table
     const bool use_small = by_rows || (srs.pre_small != nullptr && n <= small_max && offset + n <= srs.pre_small_len);
     const bool use_big = !use_small && srs.pre != nullptr && n >= ((size_t)1 << (srs.pre_c - 4));
     const bool shared = use_small || use_big;
@@ -870,34 +842,11 @@ int msm_device(jb_ctx* c, const Srs& srs, size_t offset, const void* d_scalars, 
     const size_t nb = (size_t)Weff * p.B;
     // bucket offsets, task offsets, the scatter cursor and the histogram are 32-bit: W * n sorted entries must stay
     // below 2^32 (n ~ 2^28 with 16 windows would wrap the exclusive scan and read wrong ranges - silently)
-    if ((size_t)p.W * n >= ((size_t)1 << 32) || nb + ((size_t)p.W * n) / MSM_CHUNK + 1 >= ((size_t)1 << 32))
+    const size_t entries = (size_t)p.W * n;
+    if (entries >= ((size_t)1 << 32) || nb + entries / MSM_CHUNK + 1 >= ((size_t)1 << 32))
         return c->fail(JB_ERR_UNSUPPORTED, "msm: windows x terms must be < 2^32 (split the call)");
     // upper bound on tasks: every bucket at most cnt/MSM_CHUNK + 1 chunks
-    const size_t max_tasks = nb + ((size_t)p.W * n) / MSM_CHUNK + 1;
-    // Batched-affine levels (msm_affine.cuh): field scalars only (uniform digits: a bucket holds ~entries / nb points)
-    // and only while a bucket still has several points per level. OFF by default: built, exact (tests force it at 2^13
-    // terms, exceptional pairs included) and measured SLOWER than the XYZZ accumulation it replaces - 2^24 terms,
-    // precomputed SRS: 30.6 ms of XYZZ accumulation (0.99 of the 10-products-per-addition ceiling once the tasks are
-    // walked in length order) against 35.2 / 36.2 / 38.2 ms with 2 / 3 / 4 affine levels in front of it; the level
-    // kernel reaches ~5.4 G additions/s = half of ITS ceiling (one thread's inversion idles its block, and the
-    // load - multiply - store chains of a thread expose the memory latency that the XYZZ walk hides behind 10 products).
-    // JB_MSM_BA = levels switches it on, JB_MSM_BA_MIN_LOG = log2 of the smallest windows x terms product that takes
-    // the path (tests lower it).
-    const size_t entries = (size_t)p.W * n;
-    unsigned ba_levels = 0;
-    if (kind == SK_FR && !by_rows && !use_small) {
-        const char* e_lv = getenv("JB_MSM_BA");
-        const char* e_min = getenv("JB_MSM_BA_MIN_LOG");
-        const int want = e_lv ? atoi(e_lv) : 0;
-        const int min_log = e_min ? atoi(e_min) : 26;
-        if (want > 0 && want <= 8 && entries >= ((size_t)1 << min_log)) {
-            ba_levels = (unsigned)want;
-            while (ba_levels > 0 && (entries / nb) >> ba_levels < 2) --ba_levels;  // keep >= 2 points per bucket and level
-        }
-    }
-    const size_t e_pad = entries + (ba_levels ? nb * (((size_t)1 << ba_levels) - 1) : 0);  // padded list length (bound)
-    if (e_pad >= ((size_t)1 << 32)) return c->fail(JB_ERR_UNSUPPORTED, "msm: windows x terms must be < 2^32 (split the call)");
-    uint64_t *lvl_a = nullptr, *lvl_b = nullptr, *ba_prefix = nullptr;
+    const size_t max_tasks = nb + entries / MSM_CHUNK + 1;
     uint32_t *digits = nullptr, *sorted = nullptr, *task_bucket = nullptr, *order = nullptr;
     unsigned int* len_hist = nullptr;
     unsigned int *hist = nullptr, *offsets = nullptr, *toff = nullptr, *block_sums = nullptr;
@@ -906,13 +855,7 @@ int msm_device(jb_ctx* c, const Srs& srs, size_t offset, const void* d_scalars, 
     uint64_t *tree_a = nullptr, *tree_b = nullptr;
     const size_t tree_pts = (size_t)Weff * ((p.T + 2047) / 2048) + 1;
     int st = c->dev_alloc((void**)&digits, (size_t)p.W * n * 4);
-    if (st == JB_OK) st = c->dev_alloc((void**)&sorted, e_pad * 4);
-    if (ba_levels) {
-        if (st == JB_OK) st = c->dev_alloc((void**)&lvl_a, (e_pad / 2 + 1) * 64);
-        if (st == JB_OK && ba_levels > 1) st = c->dev_alloc((void**)&lvl_b, (e_pad / 4 + 1) * 64);
-        if (st == JB_OK) st = c->dev_alloc((void**)&ba_prefix, (e_pad / 2 + 1) * 32);
-        if (st == JB_OK) st = c->check(cudaMemsetAsync(sorted, 0xFF, e_pad * 4, c->stream), "msm memset");  // holes
-    }
+    if (st == JB_OK) st = c->dev_alloc((void**)&sorted, entries * 4);
     if (st == JB_OK) st = c->dev_alloc((void**)&hist, nb * 4);
     if (st == JB_OK) st = c->dev_alloc((void**)&offsets, (nb + 1) * 4);
     if (st == JB_OK) st = c->dev_alloc((void**)&toff, (nb + 1) * 4);
@@ -936,7 +879,7 @@ int msm_device(jb_ctx* c, const Srs& srs, size_t offset, const void* d_scalars, 
             msm_digits_kernel<true><<<g, 256, 0, c->stream>>>(d_scalars, kind, d_bases, n, p.c, p.W, p.B, shared ? 1 : 0, digits, hist, row_w, halving);
         else
             msm_digits_kernel<false><<<g, 256, 0, c->stream>>>(d_scalars, kind, d_bases, n, p.c, p.W, p.B, shared ? 1 : 0, digits, hist, row_w, halving);
-        msm_scan_local_kernel<<<scan_blocks, 1024, 0, c->stream>>>(hist, offsets, toff, nb, block_sums, maxq, ba_levels);
+        msm_scan_local_kernel<<<scan_blocks, 1024, 0, c->stream>>>(hist, offsets, toff, nb, block_sums, maxq);
         msm_scan_blocks_kernel<<<1, 1024, 0, c->stream>>>(block_sums, (int)scan_blocks, offsets, toff, nb);
         msm_scan_apply_kernel<<<scan_blocks, 1024, 0, c->stream>>>(offsets, toff, nb, block_sums);
         {   // scatter, ordered in time by destination region once the destination outgrows the L2 (see the kernel)
@@ -948,10 +891,7 @@ int msm_device(jb_ctx* c, const Srs& srs, size_t offset, const void* d_scalars, 
                     regions = p.W;
                 } else if (p.c - 1 >= 6) {
                     mode = 2;
-                    int rl = 2;  // log2(regions); measured at 2^24 terms, 12 windows: 1 / 2 / 4 / 8 / 16 regions = 41.7 / 40.5 / 39.2 / 40.6 / 44.8 ms per MSM
-                    if (const char* e = getenv("JB_MSM_SCATTER_REGIONS_LOG")) rl = atoi(e);
-                    if (rl < 0) rl = 0;
-                    if (rl > 6) rl = 6;
+                    const int rl = 2;  // log2(regions); measured at 2^24 terms, 12 windows: 1 / 2 / 4 / 8 / 16 regions = 41.7 / 40.5 / 39.2 / 40.6 / 44.8 ms per MSM
                     regions = 1 << rl;
                     range_shift = (unsigned)(p.c - 1) - (unsigned)rl;  // nb = 2^(c-1) buckets
                 }
@@ -962,33 +902,12 @@ int msm_device(jb_ctx* c, const Srs& srs, size_t offset, const void* d_scalars, 
             else
                 msm_scatter_kernel<false><<<sg, 256, 0, c->stream>>>(digits, n, p.W, p.B, shared ? 1 : 0, pre_stride, offsets, hist, sorted, row_w, halving, mode, range_shift);
         }
-        int tix = c->timing_begin(4, n, p.c + 100 * (int)ba_levels);  // (window bits, affine levels) for the bench's roofline
-        const uint64_t* acc_src = d_gather;
-        for (unsigned lvl = 0; lvl < ba_levels; ++lvl) {
-            // level lvl: (e_pad >> (lvl + 1)) pairs at most (the kernel reads the exact count from offsets[nb]);
-            // pairs per thread so that ~2 blocks per SM cover the level, 8..64, even (two chains per thread)
-            const size_t pairs = e_pad >> (lvl + 1);
-            size_t kp = (pairs + (size_t)BAL_BLOCK * 296 - 1) / ((size_t)BAL_BLOCK * 296);
-            kp = kp < 8 ? 8 : kp > 64 ? 64 : kp;
-            kp += kp & 1;
-            const unsigned lg = (unsigned)((pairs + BAL_BLOCK * kp - 1) / (BAL_BLOCK * kp));
-            uint64_t* dst = (lvl & 1) ? lvl_b : lvl_a;
-            if (lvl == 0)
-                msm_affine_level_kernel<true><<<lg, BAL_BLOCK, 0, c->stream>>>(d_gather, sorted, dst, ba_prefix, offsets + nb, lvl, (unsigned)kp);
-            else
-                msm_affine_level_kernel<false><<<lg, BAL_BLOCK, 0, c->stream>>>(acc_src, nullptr, dst, ba_prefix, offsets + nb, lvl, (unsigned)kp);
-            c->launches++;
-            acc_src = dst;
-        }
-        msm_len_hist_kernel<<<MSM_TASK_BLOCKS, 256, 0, c->stream>>>(offsets, toff, nb, maxq, len_hist, ba_levels);
-        msm_tasks_kernel<<<MSM_TASK_BLOCKS, 256, 0, c->stream>>>(offsets, toff, nb, maxq, len_hist, task_bucket, order, ba_levels);
+        int tix = c->timing_begin(4, n, p.c);  // (window bits) for the bench's roofline
+        msm_len_hist_kernel<<<MSM_TASK_BLOCKS, 256, 0, c->stream>>>(offsets, toff, nb, maxq, len_hist);
+        msm_tasks_kernel<<<MSM_TASK_BLOCKS, 256, 0, c->stream>>>(offsets, toff, nb, maxq, len_hist, task_bucket, order);
         c->launches++;
-        if (ba_levels)
-            msm_accumulate_kernel<true><<<(unsigned)((max_tasks + 127) / 128), 128, 0, c->stream>>>(acc_src, sorted, offsets, toff, task_bucket,
-                                                                                                order, nb, buckets, partial, maxq, ba_levels);
-        else
-            msm_accumulate_kernel<false><<<(unsigned)((max_tasks + 127) / 128), 128, 0, c->stream>>>(d_gather, sorted, offsets, toff, task_bucket,
-                                                                                                 order, nb, buckets, partial, maxq, 0u);
+        msm_accumulate_kernel<<<(unsigned)((max_tasks + 127) / 128), 128, 0, c->stream>>>(d_gather, sorted, offsets, toff, task_bucket,
+                                                                                          order, nb, buckets, partial, maxq);
         c->timing_end(tix);
         msm_combine_kernel<<<(unsigned)((nb + 127) / 128), 128, 0, c->stream>>>(toff, nb, partial, buckets);
         if (plan_cap(maxq) > MSM_MAX_CHUNKS) {
@@ -1030,9 +949,6 @@ int msm_device(jb_ctx* c, const Srs& srs, size_t offset, const void* d_scalars, 
     c->dev_free(digits);
     c->dev_free(sorted);
     c->dev_free(task_bucket);
-    if (lvl_a) c->dev_free(lvl_a);
-    if (lvl_b) c->dev_free(lvl_b);
-    if (ba_prefix) c->dev_free(ba_prefix);
     c->dev_free(order);
     c->dev_free(len_hist);
     c->dev_free(hist);

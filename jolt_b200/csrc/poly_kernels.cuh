@@ -547,7 +547,7 @@ __device__ __forceinline__ void fused_pass(const TablePtrs& tp, size_t pairs, co
     __syncthreads();  // scratch is reused by the caller (the last block's fold)
 }
 
-// One launch per round: BLOCK threads per block (256 or 128), MINB = resident blocks per SM requested from
+// One launch per round: BLOCK threads per block, MINB = resident blocks per SM requested from
 // ptxas. WEIGHTED: the sweep is sum_y E(y) prod_j(...) with the split-eq weight E(y) = e_out * e_in folded into
 // table 0's pair AFTER the bound values are stored (GruenSplitEqPolynomial, split_eq.rs:159-447: the eq
 // polynomial is never materialised or bound as a table; its current variable is a linear factor the host
@@ -657,13 +657,11 @@ static __global__ void __launch_bounds__(256) eq_expand_kernel(const uint64_t* p
 // with a full 254-bit point this kernel is bound by the integer pipe (66.8 G mul/s x 32 B = 2.1 TB/s),
 // not by HBM.
 // CS: streaming (evict-first) stores - the table is written once and consumed by a LATER kernel; keeping 128 MB+ of
-// it dirty in L2 only evicts what the consumer wants there (A/B: tools/eq_store_probe.py, profiles/).
-// LOW3: the three register-expanded variables are the LAST three of the point, so a thread's 8 outputs are
-// CONSECUTIVE (256 B; out[(b << 11) | (t << 3) | k] = prefix[b] * mid8[t] * eq3[k], mid8 over the 8 variables before
-// them) instead of 8 KiB apart. Built to test whether the store pattern explains the 2 x DRAM write traffic ncu
-// reports for this kernel (dram__bytes_write = 2.03 x the table at 2^26): it does not - both layouts, with and
-// without streaming stores, write the same bytes (profiles/r02_eq_store_ab.md); LOW3 is 7 % slower and stays off.
-template <bool HI4, bool CS, bool LOW3 = false>
+// it dirty in L2 only evicts what the consumer wants there (A/B: profiles/r02_eq_store_ab.md).
+// Layout: a thread's 8 outputs are 8 KiB apart so that each store instruction covers 1 KiB per warp. The
+// alternative, 8 consecutive outputs per thread, writes the same DRAM bytes (2.03 x the table at 2^26 either
+// way) and measured 7 % slower (profiles/r02_eq_store_ab.md).
+template <bool HI4, bool CS>
 __global__ void __launch_bounds__(256) eq_stream_kernel(const uint64_t* prefix, const __grid_constant__ EqVars ev,
                                                         const uint64_t* low8, uint64_t* out) {
     const int tid = threadIdx.x;
@@ -679,10 +677,10 @@ __global__ void __launch_bounds__(256) eq_stream_kernel(const uint64_t* prefix, 
             e[2 * i + 1] = hi;
         }
     }
-    const size_t base = ((size_t)blockIdx.x << EQ_BLOCK_VARS) + (LOW3 ? ((size_t)tid << 3) : (size_t)tid);
+    const size_t base = ((size_t)blockIdx.x << EQ_BLOCK_VARS) + (size_t)tid;
 #pragma unroll
     for (int k = 0; k < 8; ++k) {
-        const size_t idx = base + (LOW3 ? (size_t)k : ((size_t)k << 8));
+        const size_t idx = base + ((size_t)k << 8);
         if (CS) st_elem_cs(out, idx, e[k]);
         else st_elem(out, idx, e[k]);
     }

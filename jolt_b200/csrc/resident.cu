@@ -152,9 +152,6 @@ bool resident_eligible(const jb_member* mem) {
     if (mem->len < 2 || (mem->len & (mem->len - 1))) return false;
     // a member whose big run had to make room for other work only re-enters service once its run is small
     if (mem->no_resident && mem->len > RES_SMALL_LEN) return false;
-    size_t lg = 0;
-    while (((size_t)1 << lg) < mem->len) ++lg;
-    if ((int)lg > mem->ctx->resident_max_log) return false;
     size_t smem;
     return pick_kernel(mem->m, mem->terms, mem->order, &smem) != nullptr;
 }
@@ -231,8 +228,8 @@ int resident_begin(jb_ctx* c, jb_member** mems, int n, uint64_t first_len, bool 
     std::memset(run->mb, 0, sizeof(ResMailbox));
     args.mb = (ResMailbox*)run->res.mb_dev;
     args.st = (ResState*)run->res.d_state;
-    args.timeout_cycles = c->resident_timeout_cycles;
-    args.static_pct = c->resident_static_pct;  // ~10 s of SM clocks without a command: give the SMs back
+    args.timeout_cycles = c->resident_timeout_cycles;  // ~10 s of SM clocks without a command: give the SMs back
+    args.static_pct = RES_STATIC_PCT;
     args.world = c->world;
     args.rank = c->rank;
     for (int g = 0; g < 16; ++g) args.peer[g] = c->xch_peer[g];

@@ -39,6 +39,9 @@ namespace jb {
 constexpr int RES_MAX_MEMBERS = 8;
 constexpr int RES_BLOCK = 256;
 constexpr size_t RES_SMALL_LEN = 8192;  // tables this short need few blocks: such runs coexist with other work
+// big passes: this share (%) of the pair range is laid out statically, the rest is claimed warp by warp (ResArgs::static_pct;
+// passed as an argument rather than folded in, which keeps the kernel's register allocation as measured)
+constexpr int RES_STATIC_PCT = 75;
 // Degree-2 rounds with at most this many pair indices run as THIN passes (thin_pass below): latency-shaped, and
 // they also return the lookahead sums that let the host answer the NEXT round without waiting for the device.
 constexpr uint64_t RES_THIN_PAIRS = 1ull << 17;  // (2^17: the first thin round costs what the generic pass costs there, and one more round is pipelined)

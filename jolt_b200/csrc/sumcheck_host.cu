@@ -5,7 +5,6 @@
 // The Rust toolchain is absent from this image, so the host side above the C ABI is C++ (the
 // reference is compiled code); the Rust adapter a maintainer would write is in INTEGRATION.md.
 // Everything here is O(members * rounds * degree) field work; tables never leave the device.
-#include <cstdlib>
 #include <cstring>
 #include <vector>
 
@@ -349,12 +348,12 @@ int jb_prove_batch(jb_member** members, const jb_batch_member* desc, size_t n_me
         owned.emplace_back(members[i], check_member_rounds != 0);
     }
     for (auto& m : owned) ptrs.push_back(&m);
-    // the device traversal: one host round trip per batch round (JB_SEQUENTIAL_ROUNDS=1 selects the reference's
-    // declaration-order traversal, for comparison)
+    // the device traversal: one host round trip per batch round; the reference's declaration-order traversal if
+    // the device scheduler cannot be set up
     jb::SequentialRounds seq_sched;
     jb::DeviceRoundScheduler dev_sched;
     jb::RoundScheduler* sched_ptr = &seq_sched;
-    if (!std::getenv("JB_SEQUENTIAL_ROUNDS") && n_members > 0) {
+    if (n_members > 0) {
         std::vector<jb::DeviceProductMember*> dm;
         for (auto& m : owned) dm.push_back(&m);
         jb_ctx* ctx = jb_member_context(members[0]);

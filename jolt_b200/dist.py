@@ -70,8 +70,7 @@ def init_comm(sess: Session, dist, p2p: bool = True) -> None:
     host = t.cpu().numpy().tobytes()
     buf = (ctypes.c_uint8 * 128).from_buffer_copy(host)
     sess.check(lib.jb_comm_init(sess.h, dist.get_world_size(), dist.get_rank(), buf, None))
-    import os
-    if p2p and dist.get_world_size() > 1 and not os.environ.get("JB_NO_P2P"):
+    if p2p and dist.get_world_size() > 1:
         # peer-memory exchange (CUDA IPC over NVLink): the per-round all-reduce moves into the round kernel
         world = dist.get_world_size()
         mine = (ctypes.c_uint8 * 64)()

@@ -5,15 +5,11 @@
 # tools/round_probe.py). CSVs -> gpurun_out/ (summaries are written under profiles/ on the authoring box).
 mkdir -p gpurun_out
 python tools/round_probe.py 22 2 > gpurun_out/r02_round_probe_22.txt 2>&1
-JB_NO_LOOKAHEAD=1 python tools/round_probe.py 22 2 > gpurun_out/r02_round_probe_22_nolookahead.txt 2>&1
 timeout 300 ncu --metrics gpu__time_duration.sum --clock-control none -c 800 --csv --log-file gpurun_out/r02_launches.csv \
     python bench.py --steps 2 --warmup 1 --no-cpu-baseline --no-msm --no-kernels > gpurun_out/r02_ncu_list.log 2>&1
 timeout 300 ncu --set full --clock-control none --import-source on -k regex:fused_round_kernel -c 3 -o /tmp/r02_fused \
     python bench.py --steps 1 --warmup 1 --no-cpu-baseline --no-msm --no-kernels > gpurun_out/r02_ncu_fused.log 2>&1
 ncu -i /tmp/r02_fused.ncu-rep --page raw --csv > gpurun_out/r02_fused_raw.csv 2>/dev/null
-timeout 300 ncu --set full --clock-control none --import-source on -k regex:eval2_tma_kernel -c 1 -o /tmp/r02_tma \
-    python tools/tma_ab.py 22 > gpurun_out/r02_ncu_tma.log 2>&1
-ncu -i /tmp/r02_tma.ncu-rep --page raw --csv > gpurun_out/r02_tma_raw.csv 2>/dev/null
 cat > /tmp/r02_kernels.py <<'PY'
 import sys, numpy as np
 sys.path.insert(0, "."); sys.path.insert(0, "tests")

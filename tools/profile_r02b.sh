@@ -1,8 +1,8 @@
 #!/bin/bash
 # Second-half-of-round-2 profiling on one B200 (run under gpurun from the repo root): the MSM side.
 #  * per-kernel launch list of an MSM at 2^20 and 2^24 (precomputed SRS), gpu__time_duration only;
-#  * ncu --set full of the accumulation kernel walking tasks in length order (2^22), of the batched-affine level kernel
-#    (JB_MSM_BA=2: the evidence behind "built, measured slower"), of the msm_binary select-sum kernel and of the scatter;
+#  * ncu --set full of the accumulation kernel walking tasks in length order (2^22), of the msm_binary select-sum kernel
+#    and of the scatter;
 #  * the bench's own launch list (same command as profiles/r02_launches_bench_ncu.*).
 # CSVs -> gpurun_out/ (summaries are written under profiles/ on the authoring box with tools/ncu_summary.py).
 mkdir -p gpurun_out
@@ -29,9 +29,9 @@ else:
     bases.msm(tab); bases.msm(tab)
 sess.synchronize()
 PY
-for k in acc:msm_accumulate_kernel:0:1 affine:msm_affine_level_kernel:2:2 scatter:msm_scatter_kernel:0:1 binary:msm_select_sum_kernel:0:1; do
-    IFS=: read what kern ba skip <<< "$k"   # skip: launches of the first (warm-up) MSM; affine: level 0 of the second MSM
-    JB_MSM_BA=$ba JB_MSM_BA_MIN_LOG=20 timeout 240 ncu --set full --clock-control none --import-source on -k regex:$kern -s $skip -c 1 \
+for k in acc:msm_accumulate_kernel:1 scatter:msm_scatter_kernel:1 binary:msm_select_sum_kernel:1; do
+    IFS=: read what kern skip <<< "$k"   # skip: launches of the first (warm-up) MSM
+    timeout 240 ncu --set full --clock-control none --import-source on -k regex:$kern -s $skip -c 1 \
         -o /tmp/r02b_$what python /tmp/r02b_kernels.py $what > gpurun_out/r02b_ncu_$what.log 2>&1
     ncu -i /tmp/r02b_$what.ncu-rep --page raw --csv > gpurun_out/r02b_${what}_raw.csv 2>/dev/null
 done
