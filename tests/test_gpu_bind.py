@@ -6,7 +6,7 @@ import jolt_b200
 from jolt_b200 import HIGH_TO_LOW, LOW_TO_HIGH, Polynomial
 from oracle import bn254 as O
 from oracle import coracle as C
-from gpu_util import rand_challenge, rand_full, rand_limbs
+from gpu_util import CH_ONE, CH_ZERO, parity_table, rand_challenge, rand_full, rand_limbs, rand_limbs_full, wide_hi4
 
 pytestmark = pytest.mark.gpu
 
@@ -20,10 +20,14 @@ def sess():
 
 @pytest.mark.parametrize("n", [1, 2, 5, 10, 11, 16])
 @pytest.mark.parametrize("order", [HIGH_TO_LOW, LOW_TO_HIGH])
-@pytest.mark.parametrize("kind", ["challenge125", "full254"])
+@pytest.mark.parametrize("kind", ["challenge125", "full254", "wide_hi4"])
 def test_bind_matches_oracle(sess, n, order, kind):
+    # a random half of the entries is drawn over the whole field (the top third included, which rand_limbs never
+    # reaches); wide_hi4 takes the 4-row product with hi across the top limb's whole range
     t = rand_limbs(100 + n, 1 << n)
-    r = rand_challenge(7 + n) if kind == "challenge125" else rand_full(9 + n)
+    full = np.random.Generator(np.random.PCG64(n)).integers(0, 2, size=1 << n).astype(bool)
+    t[full] = rand_limbs_full(200 + n, 1 << n)[full]
+    r = {"challenge125": rand_challenge(7 + n), "full254": rand_full(9 + n), "wide_hi4": wide_hi4(11 + n)}[kind]
     poly = Polynomial.new(sess, t)
     poly.bind_with_order(r, order)
     assert len(poly) == 1 << (n - 1)
@@ -55,6 +59,18 @@ def test_bind_edge_values_and_special_challenges(sess):
             poly.bind_with_order(r, order)
             assert (poly.evals() == C.bind(t, r, order)).all()
             poly.free()
+    # parity tables (raw r - 1 at odd popcount, pairs (0, r - 1) / (r - 1, 0)) bound with 0 (the 4-row path) and 1
+    # (the full product) select one side of every pair exactly: the result is a parity table again
+    for inv in (False, True):
+        t = parity_table(16, inv)
+        for r in (CH_ZERO, CH_ONE):
+            for order in (HIGH_TO_LOW, LOW_TO_HIGH):
+                poly = Polynomial.new(sess, t)
+                poly.bind_with_order(r, order)
+                got = poly.evals()
+                assert (got == C.bind(t, r, order, threads=4)).all()
+                assert any((got == parity_table(15, i)).all() for i in (False, True))
+                poly.free()
 
 
 def test_bind_rejects_bad_input(sess):

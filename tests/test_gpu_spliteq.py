@@ -5,12 +5,11 @@ import numpy as np
 import pytest
 
 import jolt_b200
-from jolt_b200 import (BatchMember, EqPolynomial, EqProductMember, HIGH_TO_LOW, LOW_TO_HIGH, Polynomial, ProductMember,
-                       UnivariatePoly)
+from jolt_b200 import BatchMember, EqPolynomial, EqProductMember, HIGH_TO_LOW, LOW_TO_HIGH, Polynomial, ProductMember
 from jolt_b200 import field as F
 from oracle import bn254 as O
 from oracle import coracle as C
-from gpu_util import rand_challenge, rand_limbs
+from gpu_util import rand_challenge
 
 pytestmark = pytest.mark.gpu
 
@@ -90,30 +89,29 @@ def test_eq_member_in_the_engine_and_errors(sess):
         EqProductMember(sess, [Polynomial.from_ints(sess, tabs[0])], C.ints_to_mont(w[:-1]))
 
 
-def test_eq_member_2pow18_vs_c_oracle(sess):
-    """First rounds at 2^18 against the threaded C oracle (eq table materialised on the oracle side only),
-    then the size-independent property: every round keeps s(0)+s(1)==claim and the final claim factors."""
-    n, m = 18, 2
-    thr = C.max_threads()
-    tabs = [rand_limbs(0xE9 + j, 1 << n) for j in range(m)]
-    w = rand_limbs(0x77, n)
-    gpu = EqProductMember(sess, [Polynomial.new(sess, t) for t in tabs], w)
-    cur = [C.eq_evals(w, None, thr)] + tabs
-    bind, claim = None, None
-    for rnd in range(n):
-        if rnd <= 2:
-            if bind is not None:
-                cur = [C.bind(t, bind, O.LOW_TO_HIGH, thr) for t in cur]
-            want = C.mont_to_ints(C.product_round_evals(cur, m + 1, O.LOW_TO_HIGH, thr))
-            if claim is None:
-                claim = (want[0] + want[1]) % O.R_MOD
-            got = gpu.prove_round_evals(bind, rnd, claim)
-            assert got == want
-        else:
-            got = gpu.prove_round_evals(bind, rnd, claim)
-            assert (got[0] + got[1]) % O.R_MOD == claim
-        bind = rand_challenge(3000 + rnd)
-        claim = UnivariatePoly.from_evals(got).evaluate(F.from_limbs(bind))
-    gpu.finish_rounds(bind)
-    fe = gpu.final_evals()
-    assert gpu.eq_scalar() * fe[0] * fe[1] % O.R_MOD == claim
+@pytest.mark.parametrize("order", [LOW_TO_HIGH, HIGH_TO_LOW])
+@pytest.mark.parametrize("case", ["w_zero_first", "scale_zero", "w_zero_round2"])
+def test_eq_member_noninvertible_round_is_an_error(sess, order, case):
+    """The Gruen round divides by l1 = scale * eq-so-far * w_c: a round whose l1 is zero (w_c = 0, or scale = 0) is an
+    error, not a wrong round polynomial. The rounds before it still match the oracle."""
+    n, m = 6, 2
+    tabs = [O.random_fr(40 + j, 1 << n) for j in range(m)]
+    w = O.random_fr(41, n)
+    bad_round = 2 if case == "w_zero_round2" else 0
+    if case != "scale_zero":
+        w[bad_round if order == HIGH_TO_LOW else n - 1 - bad_round] = 0   # the variable round k binds
+    scale = 0 if case == "scale_zero" else None
+    eq_tab = O.eq_evals(w, scale)
+    ref = O.ProductMember([eq_tab] + tabs, order)
+    gpu = EqProductMember(sess, [Polynomial.from_ints(sess, t) for t in tabs], C.ints_to_mont(w), scale, order=order)
+    claim = sum(e * a * b for e, a, b in zip(eq_tab, *tabs)) % O.R_MOD
+    ch = O.random_fr(42, n)
+    bind = None
+    for rnd in range(bad_round):
+        want = ref.prove_round(bind, rnd, claim)
+        got = gpu.prove_round(bind, rnd, claim)
+        assert got.coefficients == want, f"round {rnd}"
+        bind = ch[rnd]
+        claim = got.evaluate(bind)
+    with pytest.raises(jolt_b200.JoltB200Error, match="must be invertible"):
+        gpu.prove_round_evals(bind, bad_round, claim)
