@@ -129,7 +129,8 @@ int jb_eq_evals_aligned_block(jb_ctx* ctx, const uint64_t* r, size_t nvars, size
 
 /* ---- sumcheck member: ProveRounds (crates/jolt-sumcheck/src/prover.rs:52-72) for the
  *      product-of-m-tables relation, degree m (naive.rs:241-316; tests/roundtrip.rs:26-97) ------- */
-/* Takes ownership of the m tables (all the same power-of-two length). m in 1..4. */
+/* Takes ownership of the m tables (all the same power-of-two length). m in 1..8 (5..8: the wide product pass, one
+ * launch per round; see jb_scheduler_create for the degree the scheduler takes). */
 int jb_member_create(jb_ctx* ctx, const jb_table* tables, size_t m, int order, jb_member** out);
 /* Sum-of-products member: ProveRounds for  sum_x sum_{k < terms} prod_{j < factors} f_{k * factors + j}(x),
  * degree = factors, over factors * terms dense tables (term k owns tables [k * factors, (k + 1) * factors)); every
@@ -137,7 +138,7 @@ int jb_member_create(jb_ctx* ctx, const jb_table* tables, size_t m, int order, j
  * reference's optimized claim-reduction kernels after paired-eq fusion - e.g. IncClaimReduction's summand
  * A * RamInc + B * RdInc (crates/jolt-kernels/src/optimized/inc_claim_reduction.rs:47-203: factors = 2, terms = 2,
  * tables {A, RamInc, B, RdInc}); term weights are folded into one table of the term, as the reference folds gamma
- * into A and B. Built shapes: terms = 1 with factors 1..4 (== jb_member_create) and factors = 2, terms = 2.
+ * into A and B. Built shapes: terms = 1 with factors 1..8 (== jb_member_create) and factors = 2, terms = 2.
  * jb_member_final_evals returns the factors * terms bound values in table order. */
 int jb_member_create_sop(jb_ctx* ctx, const jb_table* tables, size_t factors, size_t terms, int order, jb_member** out);
 int jb_member_num_tables(jb_member* mem, size_t* tables);
@@ -163,7 +164,8 @@ int jb_member_final_evals(jb_member* mem, uint64_t* out_m_elems);
  * not-yet-current variables (two ~sqrt(N) tables), the current variable's linear factor and the hint
  * s(0)+s(1) = previous_claim complete the round polynomial on the host (gruen_poly_from_evals, :404-437).
  * w = nvars elements, w[0] <-> most significant index bit; both binding orders (LowToHigh: prefix tables
- * evals_cached, split_eq.rs:208-232; HighToLow: suffix tables evals_cached_rev, :233-257); m in 1..3; the running claim
+ * evals_cached, split_eq.rs:208-232; HighToLow: suffix tables evals_cached_rev, :233-257); m in 1..8, so the degree is at
+ * most 9 and out_evals of jb_member_prove_round takes m + 2 elements; the running claim
  * is mandatory in prove_round. Round polynomials equal those of the (m+1)-table product member over the
  * materialised eq table. jb_eq_member_scalar returns scale * eq(w, r) after the rounds. */
 int jb_eq_member_create(jb_ctx* ctx, const jb_table* tables, size_t m, const uint64_t* w, size_t nvars,
@@ -172,7 +174,8 @@ int jb_eq_member_scalar(jb_member* mem, uint64_t out[4]);
 /* Multi-GPU: like prove_round but leaves this rank's partial sums - the kernel values s(0), [s(1) unless
  * skip_t1], s(2), .., s(m-1), s(inf) in the order jb_round_evals_from_kernel_values documents - on the device as
  * count x 8 uint64 lanes, each holding one 32-bit limb (exact under ncclSum over <= 2^32 ranks); the caller
- * all-reduces that buffer, calls jb_partials_finalize and then jb_round_evals_from_kernel_values. No round check. */
+ * all-reduces that buffer, calls jb_partials_finalize and then jb_round_evals_from_kernel_values. No round check.
+ * Members of 1..4 tables only (JB_ERR_UNSUPPORTED otherwise). */
 int jb_member_prove_round_partials(jb_member* mem, const uint64_t* bind_or_null, size_t round, int skip_t1,
                                    void* device_lanes_out);
 int jb_partials_finalize(jb_ctx* ctx, const void* device_lanes, size_t count, uint64_t* out_elems);
@@ -219,7 +222,8 @@ int jb_comm_p2p_open(jb_ctx* ctx, const uint8_t* handles_world_x_64);
  * rounds and is driven by the same jb_member_prove_round / jb_prove_batch as a local member: each early
  * round costs ONE all-reduce of <= 40 u64; when a shard is 2^gather_log long the shards are
  * all-gathered once and every rank finishes the remaining rounds redundantly (identical results on all
- * ranks, identical to the single-GPU member over the global tables). `previous_claim` is the GLOBAL claim. */
+ * ranks, identical to the single-GPU member over the global tables). `previous_claim` is the GLOBAL claim.
+ * m in 1..4 (JB_ERR_UNSUPPORTED otherwise). */
 int jb_sharded_member_create(jb_ctx* ctx, const jb_table* tables, size_t m, int order, size_t gather_log,
                              jb_member** out);
 
@@ -230,7 +234,9 @@ int jb_sharded_member_create(jb_ctx* ctx, const jb_table* tables, size_t m, int 
  * it takes every round's {per-member action, shared challenge} from a mailbox in host-mapped memory and answers
  * with every member's round sums, so no kernel is launched per round; otherwise every active member's pass is
  * enqueued before the first wait (one result slot per member). `work[i].member` indexes the member list given at
- * creation; out_evals receives 8 elements (32 limbs) per work item, the first degree + 1 of them valid.
+ * creation; out_evals receives 8 elements (32 limbs) per work item, the first degree + 1 of them valid. So members
+ * of degree at most 7 only: jb_scheduler_create returns JB_ERR_UNSUPPORTED for a product of 8 tables or a split-eq
+ * member of 7 or 8 tables (jb_prove_batch then proves the batch's members in declaration order).
  * Results are identical to calling jb_member_prove_round on each item. ------------------------------------------ */
 typedef struct jb_scheduler jb_scheduler;
 typedef struct jb_round_work {   /* MemberRound, prover.rs:75-92 */

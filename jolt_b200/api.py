@@ -326,8 +326,9 @@ class UnivariatePoly:
 
 class ProductMember:
     """A device-backed ProveRounds member (prover.rs:52-72) for the relation
-    sum_x prod_j f_j(x) over m dense tables, degree m - the GPU twin of the reference tier's
-    NaiveSumcheckProver (naive.rs:241-316) / tests' DenseMember (tests.rs:1123-1175, m = 1)."""
+    sum_x prod_j f_j(x) over m = 1..8 dense tables, degree m - the GPU twin of the reference tier's
+    NaiveSumcheckProver (naive.rs:241-316) / tests' DenseMember (tests.rs:1123-1175, m = 1). A RoundScheduler takes
+    members of degree <= 7."""
 
     def __init__(self, session: Session, polys: list[Polynomial], order: int = HIGH_TO_LOW):
         self.s = session
@@ -459,7 +460,8 @@ class RoundScheduler:
 class EqProductMember(ProductMember):
     """ProveRounds member for sum_x eq(w, x) * prod_j f_j(x) (degree m + 1) with the eq polynomial kept
     split (GruenSplitEqPolynomial, crates/jolt-poly/src/split_eq.rs:159-447): no eq table is materialised,
-    bound or streamed. `w_limbs`: n elements, w[0] <-> MSB; both binding orders (split_eq.rs:208-257)."""
+    bound or streamed. `w_limbs`: n elements, w[0] <-> MSB; both binding orders (split_eq.rs:208-257). m = 1..8 tables
+    (degree up to 9); a RoundScheduler takes members of degree <= 7, i.e. m <= 6."""
 
     def __init__(self, session: Session, polys: list[Polynomial], w_limbs, scale=None, order: int = LOW_TO_HIGH):
         self.s = session

@@ -11,7 +11,7 @@
 
 #include "../../include/jolt_b200.h"
 
-constexpr int JB_MAX_EVALS = 8;                 // degree + 1 <= 8
+constexpr int JB_MAX_EVALS = 8;                 // evaluations per work item of the scheduler ABI: degree + 1 <= 8
 constexpr size_t JB_SMALL_BYTES = 4096;         // staging for round evaluations / points
 constexpr int JB_RESULT_SLOTS = 16;             // host-mapped round-result slots (1 KiB each; slot 0 = in-place rounds)
 

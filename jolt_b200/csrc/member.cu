@@ -73,7 +73,7 @@ int dispatch_weighted(jb_ctx* c, int m, int order, const TablePtrs& tp, size_t p
                            : dispatch_weighted1<2, ORDER_HIGH_TO_LOW>(c, tp, pairs, bind, hi4, s, out);
         case 3: return l2h ? dispatch_weighted1<3, ORDER_LOW_TO_HIGH>(c, tp, pairs, bind, hi4, s, out)
                            : dispatch_weighted1<3, ORDER_HIGH_TO_LOW>(c, tp, pairs, bind, hi4, s, out);
-        default: return c->fail(JB_ERR_UNSUPPORTED, "eq member: m must be 1..3");
+        default: return launch_wide_round(c, m, order, true, true, tp, pairs, bind, hi4, s, out);  // m = 4..8
     }
 }
 
@@ -96,8 +96,8 @@ int dispatch_fused1(jb_ctx* c, int order, bool skip1, const TablePtrs& tp, size_
                  : dispatch_fused2<M, P, ORDER_LOW_TO_HIGH, false>(c, tp, pairs, bind, hi4, s, out);
 }
 
-// the instantiated shapes: products of 1..4 tables; the two-term degree-2 sum of products
-bool shape_supported(int m, int terms) { return (terms == 1 && m >= 1 && m <= 4) || (terms == 2 && m == 2); }
+// the instantiated shapes: products of 1..8 tables (5..8 in wide_product.cu); the two-term degree-2 sum of products
+bool shape_supported(int m, int terms) { return (terms == 1 && m >= 1 && m <= JB_MAX_TABLES) || (terms == 2 && m == 2); }
 
 int dispatch_fused(jb_ctx* c, int m, int terms, int order, bool skip1, const TablePtrs& tp, size_t pairs, bool bind,
                    bool hi4, const BindScalar& s, const RoundOut& out) {
@@ -108,7 +108,7 @@ int dispatch_fused(jb_ctx* c, int m, int terms, int order, bool skip1, const Tab
         case 2: return dispatch_fused1<2, 1>(c, order, skip1, tp, pairs, bind, hi4, s, out);
         case 3: return dispatch_fused1<3, 1>(c, order, skip1, tp, pairs, bind, hi4, s, out);
         case 4: return dispatch_fused1<4, 1>(c, order, skip1, tp, pairs, bind, hi4, s, out);
-        default: return c->fail(JB_ERR_UNSUPPORTED, "member: m must be 1..4");
+        default: return launch_wide_round(c, m, order, skip1, false, tp, pairs, bind, hi4, s, out);  // m = 5..8
     }
 }
 
@@ -121,7 +121,7 @@ static int member_create_common(jb_ctx* c, const jb_table* handles, size_t m, si
     if (!c || !handles || !out) return JB_ERR_INVALID;
     Guard g(c);
     if (!shape_supported((int)m, (int)terms))
-        return c->fail(JB_ERR_UNSUPPORTED, "member: supported shapes are products of 1..4 tables and 2 terms x 2 factors");
+        return c->fail(JB_ERR_UNSUPPORTED, "member: supported shapes are products of 1..8 tables and 2 terms x 2 factors");
     if (order != JB_HIGH_TO_LOW && order != JB_LOW_TO_HIGH) return c->fail(JB_ERR_INVALID, "member: unknown order");
     const size_t T = m * terms;
     size_t len = 0;
@@ -295,13 +295,17 @@ static int resident_values(int D, const uint64_t* lanes, uint64_t* vals);
 static int eq_prove_round(jb_member* mem, const uint64_t* bind, size_t round, const uint64_t* claim, uint64_t* out_evals);
 
 struct RoundConsts {
-    HostFr w[4], ipow[4], mpow;
+    HostFr w[JB_MAX_TABLES], ipow[JB_MAX_TABLES], mpow;
 };
-static const RoundConsts& round_consts(int M) {  // M in 2..4
-    static RoundConsts table[5];
+static const RoundConsts& round_consts(int M) {  // M in 2..JB_MAX_TABLES
+    static RoundConsts table[JB_MAX_TABLES + 1];
     static const bool init = [] {
-        static const uint64_t binom[5][5] = {{1, 0, 0, 0, 0}, {1, 1, 0, 0, 0}, {1, 2, 1, 0, 0}, {1, 3, 3, 1, 0}, {1, 4, 6, 4, 1}};
-        for (int m = 2; m <= 4; ++m) {
+        uint64_t binom[JB_MAX_TABLES + 1][JB_MAX_TABLES + 1] = {};  // Pascal's triangle: binom[m][i] = C(m, i)
+        for (int m = 0; m <= JB_MAX_TABLES; ++m) {
+            binom[m][0] = 1;
+            for (int i = 1; i <= m; ++i) binom[m][i] = binom[m - 1][i - 1] + binom[m - 1][i];
+        }
+        for (int m = 2; m <= JB_MAX_TABLES; ++m) {
             for (int i = 0; i < m; ++i) {
                 HostFr ti = HostFr::one();  // i^m
                 for (int e = 0; e < m; ++e) ti = ti * HostFr::from_u64((uint64_t)i);
@@ -325,7 +329,7 @@ static const RoundConsts& round_consts(int M) {  // M in 2..4
 // In verify mode the claim is checked (naive.rs:301-308).
 static int assemble_evals(jb_ctx* c, int M, bool skip1, const uint64_t* vals, const uint64_t* claim, size_t round,
                           uint64_t* out_evals) {
-    HostFr ev[JB_MAX_EVALS];
+    HostFr ev[jb::JB_MEMBER_EVALS];
     int k = 0;
     ev[0] = HostFr::from_limbs(vals + 4 * k++);
     if (skip1) ev[1] = HostFr::from_limbs(claim) - ev[0];
@@ -425,7 +429,7 @@ static int run_round(jb_ctx* c, ResidentRun* run, RunItem* items, int n, const u
         else if (st != JB_OK) return st;
         else for (int i = 0; i < rn; ++i) harvest_lookahead(mems[i], info[i], out + (size_t)i * RES_SLOT_U64);
     }
-    uint64_t vals[RES_MAX_MEMBERS][JB_MAX_EVALS * 4];
+    uint64_t vals[RES_MAX_MEMBERS][jb::JB_MEMBER_EVALS * 4];
     bool hit[RES_MAX_MEMBERS], need_now = false;
     for (int i = 0; i < n && !lost; ++i) {
         jb_member* m = items[i].mem;
@@ -603,7 +607,7 @@ static int eq_prove_round(jb_member* mem, const uint64_t* bind, size_t round, co
     // kernel order: q(0), q(2), .., q(M-1), q(inf)   (M values; q(0) only for M == 1)
     const HostFr q0 = HostFr::from_limbs(c->h_result);
     const HostFr q1 = (HostFr::from_limbs(claim) - l0 * q0) * l1_inv;
-    uint64_t vals[JB_MAX_EVALS * 4], qe[JB_MAX_EVALS * 4];
+    uint64_t vals[jb::JB_MEMBER_EVALS * 4], qe[jb::JB_MEMBER_EVALS * 4];
     q0.store(vals);
     q1.store(vals + 4);
     if (M > 1) std::memcpy(vals + 8, c->h_result + 4, (M - 1) * 32);
@@ -627,7 +631,7 @@ int jb_eq_member_create(jb_ctx* c, const jb_table* handles, size_t m, const uint
                         const uint64_t* scale_or_null, int order, jb_member** out) {
     if (!c || !handles || !w || !out) return JB_ERR_INVALID;
     if (order != JB_LOW_TO_HIGH && order != JB_HIGH_TO_LOW) return c->fail(JB_ERR_INVALID, "eq member: unknown binding order");
-    if (m < 1 || m > 3) return c->fail(JB_ERR_UNSUPPORTED, "eq member: m must be 1..3");
+    if (m < 1 || m > JB_MAX_TABLES) return c->fail(JB_ERR_UNSUPPORTED, "eq member: m must be 1..8");
     for (size_t i = 0; i < nvars; ++i)
         if (!canonical_fr(w + 4 * i)) return c->fail(JB_ERR_INVALID, "eq member: point limbs not canonical");
     if (scale_or_null && !canonical_fr(scale_or_null)) return c->fail(JB_ERR_INVALID, "eq member: scale not canonical");
@@ -797,7 +801,7 @@ static int sharded_prove_round(jb_member* mem, const uint64_t* bind, size_t roun
                     if (c->h_result[0] == ~0ull && c->h_result[1] == ~0ull)
                         return c->fail(JB_ERR_CUDA, "peer exchange timed out (a rank did not arrive)");
                 }
-                uint64_t vals[JB_MAX_EVALS * 4];
+                uint64_t vals[jb::JB_MEMBER_EVALS * 4];
                 st = jb_lanes_reduce_host(c->h_result, (size_t)K, vals);
                 if (st != JB_OK) return st;
                 return assemble_evals(c, mem->m, skip1, vals, claim, round, out_evals);
@@ -838,6 +842,8 @@ int jb_sharded_member_create(jb_ctx* c, const jb_table* handles, size_t m, int o
     if (!c || !out) return JB_ERR_INVALID;
     if (!c->nccl_comm) return c->fail(JB_ERR_INVALID, "sharded member: no communicator (jb_comm_init)");
     if (order != JB_LOW_TO_HIGH && order != JB_HIGH_TO_LOW) return c->fail(JB_ERR_INVALID, "sharded member: unknown binding order");
+    // the per-round lanes and the peer exchange slots hold K <= 5 sums: sharded members stay at 1..4 tables
+    if (m < 1 || m > 4) return c->fail(JB_ERR_UNSUPPORTED, "sharded member: m must be 1..4");
     int st = jb_member_create(c, handles, m, order, out);
     if (st != JB_OK) return st;
     jb_member* mem = *out;
@@ -854,6 +860,8 @@ int jb_member_prove_round_partials(jb_member* mem, const uint64_t* bind, size_t 
     (void)round;
     if (!mem || !lanes_out) return JB_ERR_INVALID;
     Guard g(mem->ctx, true);
+    // the lanes of K <= 5 sums (K * 8 u64) are what the partials path reduces and exchanges
+    if (mem->m > 4) return mem->ctx->fail(JB_ERR_UNSUPPORTED, "partials: members of 1..4 tables only");
     before_launch(mem);
     return member_round(mem, bind, skip_t1 != 0, lanes_out);
 }
@@ -1074,6 +1082,11 @@ int jb_scheduler_create(jb_ctx* c, jb_member** members, size_t n, jb_scheduler**
                 delete s;
                 return c->fail(JB_ERR_INVALID, "scheduler: duplicate member");
             }
+        // out_evals carries JB_MAX_EVALS values per work item: a member of higher degree runs outside the scheduler
+        if ((size_t)m->m + (m->eq ? 1 : 0) + 1 > (size_t)JB_MAX_EVALS) {
+            delete s;
+            return c->fail(JB_ERR_UNSUPPORTED, "scheduler: members of degree > 7 do not fit the 8 evaluations per work item");
+        }
         s->members.push_back(m);
         if (m->sharded || m->eq || m->m != members[0]->m || m->terms != members[0]->terms || m->order != members[0]->order)
             s->homogeneous = false;
@@ -1220,7 +1233,7 @@ int jb_scheduler_prove_round(jb_scheduler* s, const jb_round_work* work, size_t 
                 if (st == JB_OK) st = wait_round_result0(c);
                 if (st == JB_OK) st = assemble_evals(c, m->m, true, c->h_result, w.claim, w.round, out_evals + i * JB_MAX_EVALS * 4);
             } else if (st == JB_OK) {
-                uint64_t vals[JB_MAX_EVALS * 4];
+                uint64_t vals[jb::JB_MEMBER_EVALS * 4];
                 answer_values(m, info[0], out, vals);
                 st = assemble_evals(c, m->m, true, vals, w.claim, w.round, out_evals + i * JB_MAX_EVALS * 4);
             }

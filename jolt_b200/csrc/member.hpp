@@ -36,6 +36,11 @@ inline bool canonical_fr(const uint64_t r[4]) { return !HostFr::geq_p(r); }
 int bind_table(jb_ctx* c, Table& t, const uint64_t r[4], int order);  // Polynomial::bind_with_order on one table
 int eq_build(jb_ctx* c, const uint64_t* r, size_t nvars, const uint64_t* scale, uint64_t* d_out);
 
+// wide_product.cu: one round of a product of m = 5..8 tables, or (weighted) of a split-eq member of m = 4..8 tables
+// (always SKIP1), with the outputs of fused_round_kernel; JB_ERR_UNSUPPORTED for any other m.
+int launch_wide_round(jb_ctx* c, int m, int order, bool skip1, bool weighted, const jb::TablePtrs& tp, size_t pairs,
+                      bool bind, bool hi4, const BindScalar& s, const jb::RoundOut& out);
+
 // Accumulates the host time spent waiting for a round result (jb_ctx_diag).
 struct WaitAcc {
     jb_ctx* c;

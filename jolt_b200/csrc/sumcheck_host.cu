@@ -98,8 +98,8 @@ int DeviceProductMember::prove_round(const HostFr* bind, size_t round, const Hos
                                      UnivariatePoly* out) {
     size_t degree = 0;
     jb_member_degree(mem_, &degree);
-    uint64_t ev[8 * 4];  // degree + 1 <= 8 (JB_MAX_EVALS)
-    if (degree + 1 > 8) return JB_ERR_UNSUPPORTED;
+    uint64_t ev[JB_MEMBER_EVALS * 4];
+    if (degree + 1 > JB_MEMBER_EVALS) return JB_ERR_UNSUPPORTED;
     int st = jb_member_prove_round(mem_, bind ? bind->l : nullptr, round, check_rounds_ ? previous_claim.l : nullptr, ev);
     if (st != JB_OK) return st;
     evals_.resize(degree + 1);

@@ -9,6 +9,9 @@
 
 namespace jb {
 
+// evaluations of one member's round: degree + 1 <= 10 (a split-eq member of 8 tables has degree 9)
+constexpr int JB_MEMBER_EVALS = 10;
+
 // jolt_poly::UnivariatePoly (crates/jolt-poly/src/univariate.rs:27-29): ascending coefficients.
 struct UnivariatePoly {
     std::vector<HostFr> coefficients;
